@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 10 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference algorithm on the host CPU cores (oracle port)
+    python bench.py --dump-outputs DIR ...    # also write what the last timed step computed, DIR/<name>.npy
 
 Prints ONE JSON line on rank 0.  Workloads (config.workload):
   train_stage2  (default) one full train_generator.py step per "step": frozen tocg -> warp -> SPADE G fwd+bwd -> D fwd+bwd
@@ -25,6 +26,7 @@ import types
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # a benchmark run leaves the tree as it found it (it may be read-only)
 
 H, W = 1024, 768
 GEN_GFLOP_PER_IMG = 1636.4  # SURVEY.md §8(d): conv FLOPs of one SPADEGenerator forward at 1024x768
@@ -108,6 +110,27 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_BYTES = 60 << 20  # --dump-outputs: all arrays together stay below 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes {name: tensor} as out_dir/<name>.npy, float64 kept and everything else as float32.  An array larger than its share of
+    DUMP_BYTES is written as a fixed sample of its flattened elements (distinct positions drawn from a generator with a constant seed,
+    so the same for the same size): two runs or two builds with the same arguments compare element for element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(arrays))
+    for name, t in arrays.items():
+        t = torch.as_tensor(t).detach()
+        t = t if t.dtype == torch.float64 else t.float()
+        k = share // t.element_size()
+        if t.numel() > k:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:k].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def build_generator(device):
     import torch
 
@@ -175,20 +198,22 @@ def cpu_baseline_gen(steps=1, warmup=0, budget_s=240.0):
 
 
 def _reference_modules():
-    """(networks, network_generator) of the UNMODIFIED reference (baseline/_ref — an untracked verbatim copy made by
-    tools/install_reference.py / __graft_entry__.build() — or /root/reference), imported under private names so that they cannot
-    be confused with this repo's drop-ins of the same file names.  None when no reference checkout travelled with the tree."""
+    """(networks, network_generator) of the UNMODIFIED reference (hrv_env.reference_dir(): the modules build() compiled into
+    oracle/_ref, or a checkout named by $HRV_REFERENCE_DIR), imported under private names so that they cannot be confused with this
+    repo's drop-ins of the same file names.  None when neither exists."""
     import importlib.util
-    for d in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.exists(os.path.join(d, "networks.py")) and os.path.exists(os.path.join(d, "network_generator.py")):
-            mods = []
-            for name in ("networks", "network_generator"):
-                spec = importlib.util.spec_from_file_location("hrv_reference_" + name, os.path.join(d, name + ".py"))
-                m = importlib.util.module_from_spec(spec)
-                spec.loader.exec_module(m)
-                mods.append(m)
-            return mods[0], mods[1], d
-    return None
+
+    import hrv_env
+    d = hrv_env.reference_dir()
+    if d is None or not all(hrv_env.reference_file(d, n) for n in ("networks", "network_generator")):
+        return None
+    mods = []
+    for name in ("networks", "network_generator"):
+        spec = importlib.util.spec_from_file_location("hrv_reference_" + name, hrv_env.reference_file(d, name))
+        m = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(m)
+        mods.append(m)
+    return mods[0], mods[1], d
 
 
 def reference_stage2_step(nets, opts, batch, h, w, opt_g, opt_d):
@@ -320,14 +345,14 @@ def host_threads():
 
 
 def cpu_baseline_train(steps=3, warmup=1, budget_s=200.0, size=(512, 384)):
-    """The reference's own modules (baseline/_ref) running one REAL train_generator.py step per timed step on the host cores: tocg
+    """The reference's own modules (oracle/_ref) running one REAL train_generator.py step per timed step on the host cores: tocg
     fwd (256x192, as in the reference) -> glue -> G fwd+bwd -> D -> hinge/feature-matching/VGG -> Adam(G) -> 2nd G fwd -> D fwd+bwd ->
     Adam(D), fp32, batch 1 at 512x384 — a quarter of the benchmarked pixel count and the smallest 4:3 size the reference generator
     admits (its latent grid is fine_width // 128 wide).  Reported as 1024x768-equivalent images/s (x 1/4: the three networks are fully
     convolutional, cost scales with pixels; the 256x192 tocg is NOT scaled down, which favours the CPU slightly).
     `warmup` / `steps` are honoured while the wall budget lasts: the loop stops early (never before one warm-up and one timed step)
     when the next step would overrun `budget_s`; what was actually run is returned and printed.  Falls back to the oracle port's
-    generator fwd+bwd (kind 'port') only when no reference checkout travelled with the tree."""
+    generator fwd+bwd (kind 'port') only when the reference modules are absent."""
     import torch
     cores = host_threads()
     torch.set_num_threads(cores)
@@ -384,7 +409,7 @@ def _cpu_baseline_port():
     out.mean().backward()
     dt = time.time() - t0
     return {"value": 0.25 / dt, "unit": "images/s", "cores": cores, "kind": "port",
-            "sample": "NO reference checkout on this box: oracle port, SPADEGenerator fwd+bwd only on one 512x384 image (%.1f s), x1/4 pixel scaling" % dt,
+            "sample": "NO reference modules (oracle/_ref): oracle port, SPADEGenerator fwd+bwd only on one 512x384 image (%.1f s), x1/4 pixel scaling" % dt,
             "s_per_step": dt, "steps_done": 1, "warmup_done": 0, "pixel_scale": 0.25}
 
 
@@ -427,7 +452,7 @@ def run_torch_gpu(args):
     import torch
     ref = _reference_modules()
     if ref is None:
-        print(json.dumps({"impl": "torch_gpu", "unavailable": "no reference checkout (baseline/_ref) on this box"}))
+        print(json.dumps({"impl": "torch_gpu", "unavailable": "no reference modules (oracle/_ref)"}))
         return
     import hrv_loader
     hrv_loader.load()
@@ -472,7 +497,11 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: per-GPU batch fixed (default 8); strong: GLOBAL batch fixed at --batch (default 8), split over the ranks")
     ap.add_argument("--dump-profile", default="", help="write the per-launch CUDA-event profile of one step as CSV")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (training: its losses and the updated parameters)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     if args.impl == "torch_gpu":
@@ -661,7 +690,7 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(k):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -669,7 +698,7 @@ def main():
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms
+        return ms, out
 
     sampler = ClockSampler(local)
     if rank == 0:
@@ -679,14 +708,21 @@ def main():
     if rank == 0:
         sampler.lines.clear()  # keep only samples taken during the timed region
     l0 = ops.LAUNCHES[0]
-    ms = timed(step_resident, K)
+    ms, out = timed(step_resident, K)
     launches = ops.LAUNCHES[0] - l0
     clocks = sampler.stop() if rank == 0 else None
     value = B * world * K / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        # before anything else runs: the steps below keep training the same parameters and reuse the graph's output buffers
+        arrays = dict(out) if isinstance(out, dict) else {"output": out}
+        if train:
+            for tag, net in ((("tocg", tocg) if stage1 else ("generator", g)), ("discriminator", D)):
+                arrays[tag + "_params"] = torch.cat([p.detach().reshape(-1).float() for p in net.parameters()])
+        dump_outputs(args.dump_outputs, arrays)
 
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, K)
+    ms_e2e, _ = timed(step_e2e, K)
     e2e_value = B * world * K / (ms_e2e / 1e3)
 
     # ---- per-kernel profile pass (CUDA events around every C-ABI launch) -> roofline of the dominant kernel

@@ -1,7 +1,7 @@
 """Environment for running the reference scripts unchanged against this repository's drop-in modules (see shims/README.md).
 
     import hrv_env; hrv_env.install()          # repo root first on sys.path, shims/ last, numpy aliases restored
-    hrv_env.load_reference_script("train_generator")   # imports baseline/_ref/train_generator.py (or /root/reference/...) with
+    hrv_env.load_reference_script("train_generator")   # imports the original train_generator (reference_dir()) with
                                                         # `networks`, `network_generator`, `sync_batchnorm` bound to the drop-ins
 """
 import importlib.util
@@ -38,9 +38,19 @@ def install():
 
 
 def reference_dir():
-    for d in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if os.path.exists(os.path.join(d, "train_generator.py")):
+    """Where the original HR-VITON modules are: the checkout named by $HRV_REFERENCE_DIR, else the compiled modules that
+    __graft_entry__.build() placed in oracle/_ref (oracle/build_reference.py), else None.  This repository does not ship them."""
+    for d in (os.environ.get("HRV_REFERENCE_DIR"), os.path.join(ROOT, "oracle", "_ref")):
+        if d and reference_file(d, "train_generator"):
             return d
+    return None
+
+
+def reference_file(d, name):
+    """<d>/<name>.py of a checkout, or the sourceless <d>/<name>.pyc of a compiled one; None when neither exists."""
+    for f in (name + ".py", name + ".pyc"):
+        if os.path.isfile(os.path.join(d, f)):
+            return os.path.join(d, f)
     return None
 
 
@@ -50,13 +60,13 @@ def load_reference_script(name, alias=None):
     install()
     d = reference_dir()
     if d is None:
-        raise FileNotFoundError("no reference checkout (baseline/_ref or /root/reference)")
+        raise FileNotFoundError("no reference modules: build with a checkout of the original HR-VITON repository, or set HRV_REFERENCE_DIR")
     import network_generator  # noqa: F401  (bind the drop-ins before the reference directory becomes importable)
     import networks  # noqa: F401
     import sync_batchnorm  # noqa: F401
     if d not in sys.path:
         sys.path.insert(1, d)  # after the repo root
-    spec = importlib.util.spec_from_file_location(alias or ("ref_" + name), os.path.join(d, name + ".py"))
+    spec = importlib.util.spec_from_file_location(alias or ("ref_" + name), reference_file(d, name))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     return mod

@@ -13,7 +13,7 @@ import torch
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "oracle"))
 import hrviton_oracle as orc  # noqa: E402
-from helpers import load_golden, synth_state_dict  # noqa: E402
+from helpers import load_golden, pick, synth_state_dict  # noqa: E402
 from hrviton_b200 import synth  # noqa: E402
 
 RATIO = 1.1          # kernels may deviate by at most this factor times the rounded oracle's own deviation (mean, tail quantile)
@@ -75,9 +75,10 @@ def tocg_floor(name, precision):
     i1, i2 = synth.tocg_inputs(n, h, w, seed)
     with torch.no_grad(), orc.storage_rounding(DT[precision]):
         flows, seg, wc, wcm = orc.tocg_forward(sd, i1, i2)
-    out = {"seg": stats(seg, g["seg"]), "warped_c": stats(wc, g["warped_c"]), "warped_cm": stats(wcm, g["warped_cm"])}
+    out = {"seg": stats(pick(g, "seg", seg), g["seg"]), "warped_c": stats(pick(g, "warped_c", wc), g["warped_c"]),
+           "warped_cm": stats(pick(g, "warped_cm", wcm), g["warped_cm"])}
     for i, f in enumerate(flows):
-        out["flow%d" % i] = stats(f, g["flow%d" % i])
+        out["flow%d" % i] = stats(pick(g, "flow%d" % i, f), g["flow%d" % i])
     return out
 
 
@@ -97,7 +98,7 @@ def gen_floor(name, precision):
 
     with torch.no_grad(), orc.storage_rounding(DT[precision]):
         out = orc.spade_generator_forward(sd, x, seg, noise)
-    return {"out": stats(out, g["out"])}
+    return {"out": stats(pick(g, "out", out), g["out"])}
 
 
 @functools.lru_cache(maxsize=None)
@@ -109,7 +110,7 @@ def gend_floor(name, precision):
     x, seg = synth.gen_inputs(n, h, w, seed, input_nc=3)
     with torch.no_grad(), orc.storage_rounding(DT[precision]):
         res = orc.gen_d_forward(sd, torch.cat([seg, x], 1))
-    return {"d%d_f%d" % (i, j): stats(f, g["d%d_f%d" % (i, j)]) for i, fs in enumerate(res) for j, f in enumerate(fs)}
+    return {"d%d_f%d" % (i, j): stats(pick(g, "d%d_f%d" % (i, j), f), g["d%d_f%d" % (i, j)]) for i, fs in enumerate(res) for j, f in enumerate(fs)}
 
 
 @functools.lru_cache(maxsize=None)

@@ -1,16 +1,19 @@
 """Generates tests/golden/*.npz by running the UNMODIFIED reference modules
-(imported from /root/reference, CPU fp32) on deterministic synthetic weights and
-inputs (hrviton_b200.synth).  Run in the build container only:
+(imported from a checkout of sangyun884/HR-VITON, CPU fp32) on deterministic synthetic
+weights and inputs (hrviton_b200.synth):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py --reference <HR-VITON checkout>
 
-The GPU box has no /root/reference; it re-creates the same weights/inputs from the
-seeds stored in each fixture and compares against the stored outputs.
+The tests need no checkout: they re-create the same weights/inputs from the seeds
+stored in each fixture and compare against the stored outputs.  Every fixture stays
+under 1 MB: an output with more than `cap` elements per image is stored as a fixed
+per-image sample (sample_large), its flat per-image indices next to it as `<key>_idx`.
 """
 import argparse
 import os
 import sys
 import types
+import zlib
 
 import numpy as np
 import torch
@@ -23,16 +26,15 @@ import hrv_loader  # noqa: E402
 hrv_loader.load()
 from hrviton_b200 import synth  # noqa: E402
 
-REF = "/root/reference"
 
-
-def import_reference():
-    sys.path.insert(0, REF)
+def import_reference(ref):
+    ref = os.path.abspath(ref)
+    sys.path.insert(0, ref)
     import importlib
     ref_networks = importlib.import_module("networks")
     ref_gen = importlib.import_module("network_generator")
-    sys.path.remove(REF)
-    assert ref_networks.__file__.startswith(REF) and ref_gen.__file__.startswith(REF)
+    sys.path.remove(ref)
+    assert ref_networks.__file__.startswith(ref) and ref_gen.__file__.startswith(ref)
     return ref_networks, ref_gen
 
 
@@ -46,18 +48,39 @@ def gen_opt(h, w):
                                  ndf=64, norm_D="spectralinstance", n_layers_D=3, num_D=2, no_ganFeat_loss=False)
 
 
+# elements per image kept of each output (sample_large), per fixture: what keeps the file under 1 MB
+CAPS = {"tocg_256x192_b1": 90112, "tocg_128x96_b2": 98304, "gen_512x384_b1": 262144, "gend_128x96_b2": 16384,
+        "gen_1024x768_b8": 28672, "tocg_1024x768_b4": 9216}
+
+
+def sample_large(arrs, cap):
+    """Floating-point outputs with more than `cap` elements per image (leading dim = batch) become (N, cap): the same `cap` positions
+    of every image, drawn once per key from a generator seeded by the key's name; their sorted flat indices are stored as `<key>_idx`
+    (tests/helpers.pick applies them to the computed output)."""
+    out = {}
+    for k, v in arrs.items():
+        a = v.detach().numpy() if torch.is_tensor(v) else np.asarray(v)
+        if cap is not None and a.dtype.kind == "f" and a.ndim > 1 and a[0].size > cap:
+            idx = np.sort(np.random.default_rng(zlib.crc32(k.encode())).choice(a[0].size, cap, replace=False)).astype(np.int32)
+            out[k + "_idx"] = idx
+            a = a.reshape(a.shape[0], -1)[:, idx]
+        out[k] = a
+    return out
+
+
 def save(name, **arrs):
     path = os.path.join(HERE, name + ".npz")
-    np.savez_compressed(path, **{k: (v.detach().numpy() if torch.is_tensor(v) else np.asarray(v)) for k, v in arrs.items()})
+    np.savez_compressed(path, **sample_large(arrs, CAPS.get(name)))
     print("wrote", path, "%.2f MB" % (os.path.getsize(path) / 1e6))
 
 
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument("--reference", required=True, help="checkout of the original HR-VITON repository")
     ap.add_argument("--only", default="")
     args = ap.parse_args()
     torch.set_num_threads(os.cpu_count())
-    ref_networks, ref_gen = import_reference()
+    ref_networks, ref_gen = import_reference(args.reference)
     torch.manual_seed(0)
 
     def want(n):

@@ -19,6 +19,19 @@ def load_golden(name):
     return {k: d[k] for k in d.files}
 
 
+def pick(g, key, t):
+    """`t` (leading dim = batch) at the positions golden `key` holds: all of them, or, where the fixture keeps a per-image sample of a
+    large output, the flat per-image indices stored beside it as `<key>_idx` (make_golden.sample_large)."""
+    idx = g.get(key + "_idx")
+    if idx is None:
+        return t
+    if torch.is_tensor(t):
+        t = t.detach().float().cpu()
+        return t.reshape(t.shape[0], -1)[:, torch.from_numpy(idx.astype(np.int64))]
+    t = np.asarray(t)
+    return t.reshape(t.shape[0], -1)[:, idx]
+
+
 def state_shapes(kind):
     with open(os.path.join(GOLDEN, "state_keys.json")) as f:
         return json.load(f)[kind]

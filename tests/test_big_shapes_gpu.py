@@ -13,7 +13,7 @@ import torch
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "..", "oracle"))
 import hrviton_oracle as orc  # noqa: E402
 import floors  # noqa: E402
-from helpers import gen_opt, load_golden, synth_state_dict, tocg_opt  # noqa: E402
+from helpers import gen_opt, load_golden, pick, synth_state_dict, tocg_opt  # noqa: E402
 from hrviton_b200 import ops, synth  # noqa: E402
 
 pytestmark = pytest.mark.gpu
@@ -38,7 +38,8 @@ def _gen_floor_image0(g, sd, x, seg, seed, n, precision):
     with torch.no_grad(), orc.storage_rounding(floors.DT[precision]):
         out = orc.spade_generator_forward(sd, x[0:1], seg[0:1], noise)
     crops = torch.stack([out[:, :, y:y + 64, x0:x0 + 64] for y, x0 in g["crop_yx"]], 1)
-    return floors.stats(out[:, :, ::8, ::8], g["sub8"][0:1].astype(np.float32)), floors.stats(crops, g["crops"][0:1].astype(np.float32))
+    return (floors.stats(pick(g, "sub8", out[:, :, ::8, ::8]), g["sub8"][0:1].astype(np.float32)),
+            floors.stats(pick(g, "crops", crops), g["crops"][0:1].astype(np.float32)))
 
 
 def test_generator_1024x768_b8(precision):
@@ -65,10 +66,11 @@ def test_generator_1024x768_b8(precision):
     assert out.shape == (n, 3, h, w) and bool(torch.isfinite(out).all())
     fl, fl_crops = _gen_floor_image0(g, sd, x, seg, seed, n, precision)
     outc = out.cpu()
-    crops = torch.stack([outc[:, :, y:y + 64, x0:x0 + 64] for y, x0 in g["crop_yx"]], 1)
+    sub8 = pick(g, "sub8", outc[:, :, ::8, ::8])
+    crops = pick(g, "crops", torch.stack([outc[:, :, y:y + 64, x0:x0 + 64] for y, x0 in g["crop_yx"]], 1))
     smax = s2max = 0.0
     for i in range(n):  # per image against the image-0 floor: same sample count on both sides of every ratio
-        s = floors.check("%s gen 1024x768 img%d sub8" % (precision, i), outc[i:i + 1, :, ::8, ::8], g["sub8"][i:i + 1].astype(np.float32), fl)
+        s = floors.check("%s gen 1024x768 img%d sub8" % (precision, i), sub8[i:i + 1], g["sub8"][i:i + 1].astype(np.float32), fl)
         s2 = floors.check("%s gen 1024x768 img%d crops" % (precision, i), crops[i:i + 1], g["crops"][i:i + 1].astype(np.float32), fl_crops)
         smax, s2max = max(smax, s["max"]), max(s2max, s2["max"])
     dmean = np.abs(outc.double().sum((2, 3)).numpy() - g["chan_sums"]) / float(h * w)
@@ -100,6 +102,7 @@ def test_tocg_1024x768_b4(precision):
     for i, f in enumerate(flows):
         items.append(("flow%d_sub" % i, f.cpu()[:, ::step(i), ::step(i)], rf[i][:, ::step(i), ::step(i)], 0.0))
     for key, got, flo, extra in items:
+        got, flo = pick(g, key, got), pick(g, key, flo)
         for i in range(n):  # image by image: local content (e.g. the 64x64 crop) sets the local error level
             fl = floors.stats(flo[i:i + 1], g[key][i:i + 1])
             s = floors.check("%s tocg 1024x768 img%d %s" % (precision, i, key), got[i:i + 1], g[key][i:i + 1], fl, extra_abs=extra)

@@ -1,7 +1,7 @@
 """The reference's OWN training loops, unmodified, on this repository's drop-in modules.
 
-`train_generator.train()` and `train_condition.train()` are imported from the reference checkout (baseline/_ref, an untracked
-verbatim copy placed there by tools/install_reference.py, or /root/reference) through hrv_env (repo root first on sys.path: `networks`,
+`train_generator.train()` and `train_condition.train()` are imported from the original HR-VITON modules that build() compiles into
+oracle/_ref (or a checkout named by $HRV_REFERENCE_DIR) through hrv_env (repo root first on sys.path: `networks`,
 `network_generator`, `sync_batchnorm` bind to the drop-ins; shims/ supplies torchgeometry / tensorboardX / apex / numpy aliases)
 and run for two iterations on a synthetic loader with the README's flags.  This is the "scripts drop in unchanged" claim of the
 boundary, exercised end to end: train-mode dispatch of ConditionGenerator / tocg-D / SPADEGenerator / gen-D forward, autograd
@@ -17,7 +17,7 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import hrv_env  # noqa: E402
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(hrv_env.reference_dir() is None, reason="no reference checkout (baseline/_ref)")]
+pytestmark = [pytest.mark.gpu, pytest.mark.skipif(hrv_env.reference_dir() is None, reason="no original HR-VITON modules: build with a checkout, or set HRV_REFERENCE_DIR")]
 
 
 class _Loader:

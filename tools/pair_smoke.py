@@ -1,5 +1,5 @@
 import os, sys, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import hrv_loader; hrv_loader.load()
 from hrviton_b200 import ops
 from hrviton_b200.ops import Act

@@ -15,7 +15,7 @@ import hrv_loader  # noqa: E402
 
 hrv_loader.load()
 import hrviton_oracle as orc  # noqa: E402
-from helpers import load_golden, synth_state_dict  # noqa: E402
+from helpers import load_golden, pick, synth_state_dict  # noqa: E402
 from hrviton_b200 import synth  # noqa: E402
 
 
@@ -34,7 +34,7 @@ def gen(name):
             return t
         with torch.no_grad(), orc.storage_rounding(dt, outs):
             out = orc.spade_generator_forward(sd, x, seg, noise)
-        d = (out.numpy() - g["out"]).__abs__()
+        d = (pick(g, "out", out).numpy() - g["out"]).__abs__()
         print("%s rounding=%s outputs=%s: max %.3e mean %.3e p99.9 %.3e" % (name, dt, outs, d.max(), d.mean(), np.quantile(d, 0.999)))
 
 
@@ -47,8 +47,7 @@ def tocg(name):
     for dt, outs in ((None, True), (torch.bfloat16, True), (torch.bfloat16, False), (torch.float16, True)):
         with torch.no_grad(), orc.storage_rounding(dt, outs):
             flows, seg, wc, wcm = orc.tocg_forward(sd, i1, i2)
-        rows = [("seg", seg, g["seg"]), ("warped_c", wc, g["warped_c"]), ("warped_cm", wcm, g["warped_cm"])] + \
-               [("flow%d" % i, f, g["flow%d" % i]) for i, f in enumerate(flows)]
+        rows = [(k, pick(g, k, t), g[k]) for k, t in [("seg", seg), ("warped_c", wc), ("warped_cm", wcm)] + [("flow%d" % i, f) for i, f in enumerate(flows)]]
         print("%s rounding=%s outputs=%s: " % (name, dt, outs) + "  ".join("%s max %.2e mean %.2e" % (k, np.abs(a.numpy() - b).max(), np.abs(a.numpy() - b).mean()) for k, a, b in rows))
 
 
