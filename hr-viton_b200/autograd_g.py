@@ -1,4 +1,4 @@
-"""Training path (forward + backward) of the SPADE generator and its discriminator.
+"""Training path (forward + backward) of the SPADE generator, and the one forward of both PatchGAN discriminators.
 
 torch.autograd carries the graph; every node is a fused C-ABI op on pixel-major bf16 buffers:
 
@@ -18,9 +18,8 @@ import torch
 import torch.nn.functional as F
 
 from . import ops
-from .ops import ACT_LRELU, ACT_NONE, ACT_RELU, ACT_TANH, Act
-
-_PACK_DTYPE = torch.bfloat16
+from .ops import ACT_LRELU, ACT_NONE, ACT_RELU, ACT_TANH, Act, im2col_weight
+from .spade import conv_weight
 
 
 def _act_grad(dy, y, act):
@@ -189,15 +188,8 @@ class FromNCHW(torch.autograd.Function):
         return Act(dbuf.contiguous(), c=c).to_nchw(), None, None
 
 
-def im2col_weight(w, k_pad):
-    """(cout,cin,kh,kw) -> (cout,k_pad,1,1) in the tap-major column order of hrv_im2col (differentiable index shuffle)."""
-    cout, cin, kh, kw = w.shape
-    return F.pad(w.permute(0, 2, 3, 1).reshape(cout, kh * kw * cin), (0, k_pad - kh * kw * cin)).reshape(cout, k_pad, 1, 1)
-
-
 def _block_train(blk, x0_buf, x0_shift, x1_buf, seg_buf, noise_fn, out_act):
     """SPADEResBlock forward with autograd nodes (network_generator.py:157-173)."""
-    from .spade import _conv_weight_train
     n, h, w, _ = seg_buf.shape
     seg_c = blk.norm_0.conv_shared[0].weight.shape[1]
     # 3x3 over the few-channel label map: gather the 9 taps once per block (shared by its 2-3 norms) so each mlp_shared
@@ -219,14 +211,14 @@ def _block_train(blk, x0_buf, x0_shift, x1_buf, seg_buf, noise_fn, out_act):
         st_s, st_0 = ops.instnorm_stats2(Act(x0_buf), x0_shift, Act(x1_buf) if x1_buf is not None else None, h, w, [nz_s, nz_0],
                                          [blk.norm_s.noise_scale.detach().float().contiguous(), blk.norm_0.noise_scale.detach().float().contiguous()])
         hs = spade(blk.norm_s, x0_buf, x0_shift, x1_buf, ACT_NONE, nz_s, st_s)
-        x_s = conv(hs, _conv_weight_train(blk.conv_s, blk.training))
+        x_s = conv(hs, conv_weight(blk.conv_s, blk.training))
         h0 = spade(blk.norm_0, x0_buf, x0_shift, x1_buf, ACT_LRELU, nz_0, st_0)
     else:
         x_s = x0_buf
         h0 = spade(blk.norm_0, x0_buf, x0_shift, x1_buf, ACT_LRELU)
-    dx = conv(h0, _conv_weight_train(blk.conv_0, blk.training), blk.conv_0.bias)
+    dx = conv(h0, conv_weight(blk.conv_0, blk.training), blk.conv_0.bias)
     h1 = spade(blk.norm_1, dx, 0, None, ACT_LRELU)
-    return conv(h1, _conv_weight_train(blk.conv_1, blk.training), blk.conv_1.bias, res_buf=x_s, act=out_act)
+    return conv(h1, conv_weight(blk.conv_1, blk.training), blk.conv_1.bias, res_buf=x_s, act=out_act)
 
 
 def generator_forward_train(g, x, seg):
@@ -250,7 +242,7 @@ def generator_forward_train(g, x, seg):
     return conv(h, g.conv_img.weight, g.conv_img.bias, act=ACT_TANH, out_fp32_nchw=True)
 
 
-# ------------------------------------------------------------------------------------------------ discriminator (training)
+# ------------------------------------------------------------------------------------------------ discriminator
 
 class S2DFn(torch.autograd.Function):
     """Space-to-depth by 2 with zero fill of odd edges, channel order (py*2+px)*C8 + c (hrv_space_to_depth / ops.s2d_weight
@@ -325,48 +317,55 @@ class InstNormActFn(torch.autograd.Function):
         return dx.buf, None
 
 
-def _nlayer_train(d, x_buf, need_wgrad):
-    """One NLayerDiscriminator (network_generator.py:250-291) on a pixel-major input; returns the per-group outputs."""
-    from .spade import _conv_weight_train
+def patchgan_forward(seqs, x_buf, training, need_wgrad=True):
+    """PatchGAN discriminator layers (network_generator.py:250-291, networks.py:351-408) on a pixel-major input.  Each nn.Sequential
+    (nested ones flattened) chains Conv2d 4x4 (stride 2 | 1, pad 2), each followed by an optional InstanceNorm2d, an optional LeakyReLU
+    and an optional Dropout, and runs on the previous one's output.  Returns each sequence's output buffer (fp32 for the 1-channel
+    last layer).  need_wgrad=False detaches the weights (D inside the G step)."""
     outs = []
     h = x_buf
-    for i in range(d.n_groups):
-        first = getattr(d, "model%d" % i)[0]
-        convm = first[0] if isinstance(first, torch.nn.Sequential) else first
-        has_in = isinstance(first, torch.nn.Sequential) and d._instance
-        w = _conv_weight_train(convm, d.training)
-        if not need_wgrad:
-            w = w.detach()
-        bias = getattr(convm, "bias", None)
-        if bias is not None and not need_wgrad:
-            bias = bias.detach()
-        last = i == d.n_groups - 1
-        if convm.stride[0] == 2:
-            w2 = ops.s2d_weight(w, 2) if not w.requires_grad else _s2d_weight_t(w)
-            src = space_to_depth_t(h, w.shape[1])
-            # k4 s2 p2 on (H,W) == k2 s1 p1 on the space-to-depth tensor; extent floor(H/2)+1 (one less than the s2d conv's
-            # natural extent when H is odd: the kernels simply do not compute / read the cropped row)
-            y = conv(src, w2, bias, act=ACT_NONE if has_in else ACT_LRELU, pad=1, out_hw=(h.shape[1] // 2 + 1, h.shape[2] // 2 + 1))
-        else:
-            y = conv(h, w, bias, pad=2, out_f32_nhwc=last)
-        if has_in:
-            y = InstNormActFn.apply(y, ACT_LRELU)
-        outs.append(y)
-        h = y
+    for seq in seqs:
+        mods = [m for m in seq.modules() if not isinstance(m, torch.nn.Sequential)]
+        j = 0
+        while j < len(mods):
+            m = mods[j]
+            if isinstance(m, torch.nn.Conv2d):
+                nxt = mods[j + 1:j + 3]
+                if nxt and isinstance(nxt[0], torch.nn.BatchNorm2d):
+                    raise NotImplementedError("BatchNorm discriminators have no kernel (the reference uses norm='instance')")
+                has_in = bool(nxt) and isinstance(nxt[0], torch.nn.InstanceNorm2d)
+                has_lr = len(nxt) > has_in and isinstance(nxt[has_in], torch.nn.LeakyReLU)
+                w, bias = conv_weight(m, training), m.bias
+                if not need_wgrad:
+                    w, bias = w.detach(), (bias.detach() if bias is not None else None)
+                act = ACT_LRELU if (has_lr and not has_in) else ACT_NONE
+                if m.stride[0] == 2:
+                    # k4 s2 p2 on (H,W) == k2 s1 p1 on the space-to-depth tensor; extent floor(H/2)+1 (one less than the s2d conv's
+                    # natural extent when H is odd: the kernels simply do not compute / read the cropped row)
+                    y = conv(space_to_depth_t(h, w.shape[1]), ops.s2d_weight(w, 2), bias, act=act, pad=1,
+                             out_hw=(h.shape[1] // 2 + 1, h.shape[2] // 2 + 1))
+                else:
+                    y = conv(h, w, bias, act=act, pad=2, out_f32_nhwc=w.shape[0] == 1)
+                h = InstNormActFn.apply(y, ACT_LRELU if has_lr else ACT_NONE) if has_in else y
+                j += 1 + has_in + has_lr
+            elif isinstance(m, torch.nn.Dropout):
+                h = F.dropout(h, m.p, training)
+                j += 1
+            elif isinstance(m, torch.nn.Sigmoid):
+                raise NotImplementedError("use_sigmoid=True has no kernel (the reference uses LSGAN, use_sigmoid=False)")
+            else:
+                raise NotImplementedError("unexpected layer %s in a PatchGAN sequence" % type(m).__name__)
+        outs.append(h)
     return outs
 
 
-def _s2d_weight_t(w):
-    """Differentiable version of ops.s2d_weight (index shuffle only): k=4/pad=2, or k=3/pad=1 embedded in a 4x4 kernel with a
-    zero first row/column (tap ky of the 3x3 sits at ky+1)."""
-    if w.shape[2] == 3:
-        w = F.pad(w, (1, 0, 1, 0))
-    cout, cin, k, _ = w.shape
-    assert k == 4
-    cin8 = ops.round_up(cin, 8)
-    wp = F.pad(w, (0, 0, 0, 0, 0, cin8 - cin))                      # (cout, cin8, 4, 4)
-    wp = wp.reshape(cout, cin8, 2, 2, 2, 2)                          # ky = ty*2+py, kx = tx*2+px
-    return wp.permute(0, 3, 5, 1, 2, 4).reshape(cout, 4 * cin8, 2, 2)  # channel = (py*2+px)*cin8 + ci, taps (ty,tx)
+def nchw(buf, as_float=True):
+    """NCHW form of a pixel-major output: while autograd records, the differentiable permuted view (fp32 when as_float); otherwise a
+    contiguous fp32 copy (hrv_nhwc_to_nchw)."""
+    if not torch.is_grad_enabled():
+        return Act(buf).to_nchw()
+    v = buf.permute(0, 3, 1, 2)
+    return v.float() if as_float else v
 
 
 class FeatMatchFn(torch.autograd.Function):
@@ -395,24 +394,15 @@ class FeatMatchFn(torch.autograd.Function):
 
 
 def discriminator_forward_train(D, input_nchw, need_wgrad=True, as_float=True, raw=False):
-    """MultiscaleDiscriminator.forward with autograd (network_generator.py:293-316); returns NCHW fp32 feature lists
+    """MultiscaleDiscriminator.forward (network_generator.py:293-316); returns NCHW feature lists (see nchw)
     (raw=True: the pixel-major buffers themselves for the intermediate features — FeatMatchFn's operand — and the NCHW view of the
     last, 1-channel output)."""
-    x = FromNCHW.apply(input_nchw, None, None)
-    cin = input_nchw.shape[1]
+    cur = FromNCHW.apply(input_nchw, None, None)
     result = []
     ds = list(D.children())
-    cur = x
     for k, d in enumerate(ds):
-        outs = _nlayer_train(d, cur, need_wgrad)
-        feats = []
-        for j, o in enumerate(outs):
-            if raw and j + 1 < len(outs):
-                feats.append(o)
-                continue
-            c = o.shape[3] if o.dtype != torch.float32 else 1
-            v = o[..., :c].permute(0, 3, 1, 2)  # NCHW view of the pixel-major buffer (no copy)
-            feats.append(v.float() if as_float else v)
+        outs = patchgan_forward(list(d.children()), cur, d.training, need_wgrad)
+        feats = [o if raw and j + 1 < len(outs) else nchw(o, as_float) for j, o in enumerate(outs)]
         result.append(feats if not D.no_ganFeat_loss else [feats[-1]])
         if k + 1 < len(ds):
             cur = AvgPool3S2Fn.apply(cur)

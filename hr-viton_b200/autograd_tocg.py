@@ -8,8 +8,8 @@ import torch
 import torch.nn.functional as F
 
 from . import ops
-from .autograd_g import AvgPool3S2Fn, FromNCHW, InstNormActFn, conv, space_to_depth_t, _s2d_weight_t
-from .ops import ACT_LRELU, ACT_NONE, ACT_RELU, Act
+from .autograd_g import AvgPool3S2Fn, FromNCHW, conv, nchw, patchgan_forward, space_to_depth_t
+from .ops import ACT_RELU, Act
 
 
 class BatchNormActFn(torch.autograd.Function):
@@ -108,7 +108,7 @@ def _resblock(rb, x_buf):
         w = rb.scale.weight
         src = space_to_depth_t(x_buf, w.shape[1])
         oh, ow = (x_buf.shape[1] - 1) // 2 + 1, (x_buf.shape[2] - 1) // 2 + 1  # k3 s2 p1 extent; the s2d form would give one more
-        r = conv(src, _s2d_weight_t(w), rb.scale.bias, pad=1, out_hw=(oh, ow))
+        r = conv(src, ops.s2d_weight(w, 1), rb.scale.bias, pad=1, out_hw=(oh, ow))
     elif rb.kind == "same":
         r = conv(x_buf, rb.scale.weight, rb.scale.bias, pad=0)
     else:
@@ -116,26 +116,6 @@ def _resblock(rb, x_buf):
     bn0, bn1 = rb.block[1], rb.block[4]
     h = BatchNormActFn.apply(conv(r, rb.block[0].weight, rb.block[0].bias), bn0.weight, bn0.bias, None, bn0, ACT_RELU)
     return BatchNormActFn.apply(conv(h, rb.block[3].weight, rb.block[3].bias), bn1.weight, bn1.bias, r, bn1, ACT_RELU)
-
-
-_GRIDS = {}
-
-
-def _base_grid(n, h, w, device):
-    key = (n, h, w, str(device))
-    if key not in _GRIDS:
-        gx = torch.linspace(-1.0, 1.0, w).view(1, 1, w, 1).expand(n, h, w, 1)
-        gy = torch.linspace(-1.0, 1.0, h).view(1, h, 1, 1).expand(n, h, w, 1)
-        _GRIDS[key] = torch.cat([gx, gy], 3).to(device)
-    return _GRIDS[key]
-
-
-def _warp(src_nchw, flow_lo):
-    """networks.py:133-135 / 147-152: flow x2 (bilinear), normalise by ((W/2-1)/2,(H/2-1)/2), + base grid, grid_sample(border)."""
-    n, _, h, w = src_nchw.shape
-    fl = F.interpolate(flow_lo.permute(0, 3, 1, 2), scale_factor=2, mode="bilinear", align_corners=False).permute(0, 2, 3, 1)
-    fn = torch.cat([fl[..., 0:1] / ((w / 2 - 1.0) / 2.0), fl[..., 1:2] / ((h / 2 - 1.0) / 2.0)], 3)
-    return F.grid_sample(src_nchw, fn + _base_grid(n, h, w, src_nchw.device), mode="bilinear", padding_mode="border", align_corners=False), fl
 
 
 def tocg_forward_train(m, input1, input2):
@@ -176,48 +156,20 @@ def tocg_forward_train(m, input1, input2):
 
 # ------------------------------------------------------------------------------------------------ stage-1 discriminator
 
-def _patch_sequence_train(seq, h, training):
-    """nn.Sequential of {Conv2d 4x4 (s2|s1, pad 2), InstanceNorm2d, LeakyReLU, Dropout} (networks.py:351-408) with autograd nodes."""
-    from .spade import _conv_weight_train
-    mods = list(seq)
-    j = 0
-    while j < len(mods):
-        mod = mods[j]
-        if isinstance(mod, torch.nn.Conv2d):
-            nxt = mods[j + 1:j + 3]
-            has_in = len(nxt) > 0 and isinstance(nxt[0], torch.nn.InstanceNorm2d)
-            has_lr = any(isinstance(q, torch.nn.LeakyReLU) for q in nxt[:2])
-            w = _conv_weight_train(mod, training)
-            last = w.shape[0] == 1
-            fused_act = ACT_LRELU if (has_lr and not has_in) else ACT_NONE
-            if mod.stride[0] == 2:
-                oh, ow = h.shape[1] // 2 + 1, h.shape[2] // 2 + 1
-                y = conv(space_to_depth_t(h, w.shape[1]), _s2d_weight_t(w), mod.bias, act=fused_act, pad=1, out_hw=(oh, ow))
-            else:
-                y = conv(h, w, mod.bias, act=fused_act, pad=2, out_f32_nhwc=last)
-            if has_in:
-                y = InstNormActFn.apply(y, ACT_LRELU if has_lr else ACT_NONE)
-            h = y
-            j += 1 + int(has_in) + int(has_lr)
-        elif isinstance(mod, torch.nn.Dropout):
-            h = F.dropout(h, mod.p, training)
-            j += 1
-        else:
-            raise NotImplementedError("unexpected layer %s in a PatchGAN sequence" % type(mod).__name__)
-    return h
-
-
 def tocg_discriminator_forward_train(D, input_nchw):
-    """networks.MultiscaleDiscriminator.forward (networks.py:331-349), getIntermFeat=False: list[num_D] of [logits NCHW fp32]."""
-    if D.getIntermFeat:
-        raise NotImplementedError("getIntermFeat=True training path is not built (the reference trains with getIntermFeat=False)")
+    """networks.MultiscaleDiscriminator.forward (networks.py:331-349): list[num_D] of NCHW fp32 feature lists (see autograd_g.nchw), the
+    per-layer features with getIntermFeat, else [logits]."""
     buf = FromNCHW.apply(input_nchw.float(), None, None)
     if D.Ddownx2:
         buf = AvgPool3S2Fn.apply(buf)
     res = []
     for i in range(D.num_D):
-        o = _patch_sequence_train(getattr(D, "layer%d" % (D.num_D - 1 - i)), buf, D.training)
-        res.append([o.permute(0, 3, 1, 2)])
+        k = D.num_D - 1 - i
+        if D.getIntermFeat:
+            seqs = [getattr(D, "scale%d_layer%d" % (k, j)) for j in range(D.n_layers + 2)]
+        else:
+            seqs = [getattr(D, "layer%d" % k)]
+        res.append([nchw(o) for o in patchgan_forward(seqs, buf, D.training)])
         if i != D.num_D - 1:
             buf = AvgPool3S2Fn.apply(buf)
     return res

@@ -3,6 +3,7 @@ import ctypes
 from dataclasses import dataclass
 
 import torch
+import torch.nn.functional as F
 
 from . import capi
 from .capi import ACT_LRELU, ACT_NONE, ACT_RELU, ACT_TANH, BF16, F32  # noqa: F401
@@ -215,19 +216,20 @@ def pack_weight(w, off, cin_total=None, interleave=None, bn=None, flops_per_pixe
 
 def s2d_weight(w, pad):
     """Rewrite a stride-2 conv weight (Cout,Cin,k,k) with padding `pad` (k=4,pad=2 or k=3,pad=1) as the
-    2x2 stride-1 weight over the space-to-depth input with channel order (py*2+px)*Cin8 + ci, off=(1,1)."""
+    2x2 stride-1 weight over the space-to-depth input with channel order (py*2+px)*Cin8 + ci, off=(1,1).
+    An index shuffle, so gradients flow back to w.  The 3x3 form is the 4x4 one with a zero first row/column
+    (tap ky of the 3x3 sits at ky+1)."""
     cout, cin, k, _ = w.shape
-    cin8 = round_up(cin, 8)
-    out = torch.zeros((cout, 4 * cin8, 2, 2), dtype=w.dtype, device=w.device)
-    shift = 0 if (k == 4 and pad == 2) else 1
     assert (k, pad) in ((4, 2), (3, 1))
-    for ky in range(k):
-        ty, py = divmod(ky + shift, 2)
-        for kx in range(k):
-            tx, px = divmod(kx + shift, 2)
-            sub = py * 2 + px
-            out[:, sub * cin8:sub * cin8 + cin, ty, tx] = w[:, :, ky, kx]
-    return out
+    cin8 = round_up(cin, 8)
+    wp = F.pad(w, (4 - k, 0, 4 - k, 0, 0, cin8 - cin)).reshape(cout, cin8, 2, 2, 2, 2)  # ky = ty*2+py, kx = tx*2+px
+    return wp.permute(0, 3, 5, 1, 2, 4).reshape(cout, 4 * cin8, 2, 2)  # channel = (py*2+px)*cin8 + ci, taps (ty,tx)
+
+
+def im2col_weight(w, k_pad):
+    """(cout,cin,kh,kw) -> (cout,k_pad,1,1) in the tap-major column order of hrv_im2col (differentiable index shuffle)."""
+    cout, cin, kh, kw = w.shape
+    return F.pad(w.permute(0, 2, 3, 1).reshape(cout, kh * kw * cin), (0, k_pad - kh * kw * cin)).reshape(cout, k_pad, 1, 1)
 
 
 def pack_s2d(w, pad):

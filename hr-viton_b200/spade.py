@@ -84,39 +84,29 @@ class MaskNorm(nn.Module):
         raise NotImplementedError("MaskNorm is dead code in the reference generator and is out of scope (SURVEY.md §2 row 7)")
 
 
+def _records_grad(module, x):
+    """Whether a forward of `module` on `x` has to build an autograd graph."""
+    return torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in module.parameters()))
+
+
 def _sigma(conv, training):
     """Old-style torch spectral_norm (dim 0, 1 power iteration, eps 1e-12): in training mode u,v are refreshed in
-    place without grad, sigma = u . (W v) (network_generator.py:138-143; SURVEY.md §8 B5)."""
-    w = conv.weight_orig.detach()
-    wm = w.reshape(w.shape[0], -1)
+    place without grad, sigma = u . (W v) with the gradient through W (network_generator.py:138-143; SURVEY.md §8 B5).
+    u and v enter as copies: the next forward's refresh must not invalidate a graph still waiting for its backward."""
+    wm = conv.weight_orig.reshape(conv.weight_orig.shape[0], -1)
     u, v = conv.weight_u, conv.weight_v
     if training:
         with torch.no_grad():
             v.copy_(torch.nn.functional.normalize(torch.mv(wm.t(), u), dim=0, eps=1e-12))
             u.copy_(torch.nn.functional.normalize(torch.mv(wm, v), dim=0, eps=1e-12))
-    return torch.dot(u, torch.mv(wm, v))
+    return torch.dot(u.detach().clone(), torch.mv(wm, v.detach().clone()))
 
 
-def _conv_weight(conv, training):
-    """Effective fp32 weight of a (possibly spectrally normalised) conv container."""
+def conv_weight(conv, training):
+    """Effective fp32 weight of a conv container: W_orig / sigma when it is spectrally normalised, else its weight.
+    Differentiable; inference callers detach it."""
     if hasattr(conv, "weight_orig"):
-        return conv.weight_orig.detach() / _sigma(conv, training)
-    return conv.weight.detach()
-
-
-def _conv_weight_train(conv, training):
-    """Differentiable effective weight: W_orig / sigma with sigma = u.(W v) carrying the gradient through W (u, v are
-    buffers refreshed in place by one power iteration in training mode) — torch spectral_norm semantics."""
-    if hasattr(conv, "weight_orig"):
-        w = conv.weight_orig
-        wm = w.reshape(w.shape[0], -1)
-        u, v = conv.weight_u, conv.weight_v
-        if training:
-            with torch.no_grad():
-                v.copy_(torch.nn.functional.normalize(torch.mv(wm.t(), u), dim=0, eps=1e-12))
-                u.copy_(torch.nn.functional.normalize(torch.mv(wm, v), dim=0, eps=1e-12))
-        sigma = torch.dot(u.detach().clone(), torch.mv(wm, v.detach().clone()))
-        return w / sigma
+        return conv.weight_orig / _sigma(conv, training)
     return conv.weight
 
 
@@ -194,20 +184,19 @@ class SPADEResBlock(nn.Module):
             if 9 * wsh.shape[1] <= 64:
                 # few-channel label map: column (im2col) form, one K=64 block instead of nine K=16 taps; one 128-channel GEMM per
                 # norm (<= 128 output channels keeps each on the pixel-N kernel) writing its slice of the shared actv buffer
-                from .autograd_g import im2col_weight
-                shared = [ops.pack_weight(im2col_weight(m.conv_shared[0].weight.detach(), 64), (0, 0),
+                shared = [ops.pack_weight(ops.im2col_weight(m.conv_shared[0].weight.detach(), 64), (0, 0),
                                           flops_per_pixel=2.0 * m.conv_shared[0].weight.shape[0] * wsh.shape[1] * 9) for m in norms]
             else:
                 shared = ops.pack_weight(wsh, (1, 1))
             c = {"shared": shared,
                  "shared_b": torch.cat([m.conv_shared[0].bias.detach() for m in norms], 0).float().contiguous(),
                  "n0": self.norm_0.packed(), "n1": self.norm_1.packed(),
-                 "c0": ops.pack_weight(_conv_weight(self.conv_0, self.training), (1, 1)),
-                 "c1": ops.pack_weight(_conv_weight(self.conv_1, self.training), (1, 1)),
+                 "c0": ops.pack_weight(conv_weight(self.conv_0, self.training).detach(), (1, 1)),
+                 "c1": ops.pack_weight(conv_weight(self.conv_1, self.training).detach(), (1, 1)),
                  "b0": self.conv_0.bias.detach().float().contiguous(), "b1": self.conv_1.bias.detach().float().contiguous()}
             if self.learned_shortcut:
                 c["ns"] = self.norm_s.packed()
-                c["cs"] = ops.pack_weight(_conv_weight(self.conv_s, self.training), (0, 0))
+                c["cs"] = ops.pack_weight(conv_weight(self.conv_s, self.training).detach(), (0, 0))
             self._cache, self._cache_key = c, (_param_key(self), self.training)
         return self._cache
 
@@ -382,7 +371,6 @@ class NLayerDiscriminator(BaseNetwork):
         self.no_ganFeat_loss = opt.no_ganFeat_loss
         nf = opt.ndf
         norm_layer = get_nonspade_norm_layer(opt.norm_D)
-        self._instance = "instance" in opt.norm_D
         if "batch" in opt.norm_D:
             raise NotImplementedError("norm_D with BatchNorm has no kernel; the reference uses 'spectralinstance'")
         input_nc = opt.gen_semantic_nc + 3
@@ -393,54 +381,13 @@ class NLayerDiscriminator(BaseNetwork):
         groups.append([nn.Conv2d(nf, 1, kernel_size=4, stride=1, padding=2)])
         for i, g in enumerate(groups):
             self.add_module("model" + str(i), nn.Sequential(*g))
-        self.n_groups = len(groups)
-        self._cache_key = None
-        self._cache = None
-
-    def _packed(self):
-        key = (_param_key(self), self.training)
-        if key != self._cache_key or self.training:
-            packs = []
-            for i in range(self.n_groups):
-                first = getattr(self, "model%d" % i)[0]
-                conv = first[0] if isinstance(first, nn.Sequential) else first
-                w = _conv_weight(conv, self.training)
-                bias = conv.bias.detach().float().contiguous() if getattr(conv, "bias", None) is not None else None
-                if conv.stride[0] == 2:
-                    pw = ops.pack_s2d(w, 2)
-                else:
-                    pw = ops.pack_weight(w, (2, 2))
-                packs.append((pw, bias, conv.stride[0], isinstance(first, nn.Sequential) and self._instance))
-            self._cache, self._cache_key = packs, (_param_key(self), self.training)
-        return self._cache
-
-    def run(self, a):
-        """a: pixel-major bf16 input. Returns the list of per-group outputs as Acts (last one fp32, 1 channel)."""
-        outs = []
-        for i, (pw, bias, stride, has_in) in enumerate(self._packed()):
-            last = i == self.n_groups - 1
-            if stride == 2:
-                src = ops.space_to_depth(a)
-                oh, ow = a.h // 2 + 1, a.w // 2 + 1  # k4 s2 p2: floor(h/2)+1 (the extra row reads TMA zero fill)
-            else:
-                src, oh, ow = a, a.h + 1, a.w + 1
-            if last:
-                o = Act.empty(a.n, oh, ow, 1, dtype=torch.float32, pitch=1)
-                ops.conv2d(src, pw, o, shift=bias)
-            elif has_in:
-                o = ops.conv2d(src, pw, Act.empty(a.n, oh, ow, pw.n_gemm), shift=bias)
-                mean, rstd = ops.instnorm_stats(o, 0, None, oh, ow, None, None)
-                ops.instnorm_apply(o, mean, rstd, ACT_LRELU)
-            else:
-                o = ops.conv2d(src, pw, Act.empty(a.n, oh, ow, pw.n_gemm), shift=bias, act=ACT_LRELU)
-            outs.append(o)
-            a = o
-        return outs
 
     def forward(self, input):
         _need_cuda(input, "NLayerDiscriminator")
-        with torch.no_grad():
-            res = [o.to_nchw() for o in self.run(ops.from_nchw(input.float()))]
+        from . import autograd_g
+        with torch.set_grad_enabled(_records_grad(self, input)):
+            outs = autograd_g.patchgan_forward(list(self.children()), autograd_g.FromNCHW.apply(input.float(), None, None), self.training)
+            res = [autograd_g.nchw(o) for o in outs]
         return res if not self.no_ganFeat_loss else res[-1]
 
 
@@ -459,22 +406,9 @@ class MultiscaleDiscriminator(BaseNetwork):
 
     def forward(self, input):
         _need_cuda(input, "MultiscaleDiscriminator")
-        if torch.is_grad_enabled() and (input.requires_grad or any(p.requires_grad for p in self.parameters())):
-            try:
-                from . import autograd_g
-            except ImportError:
-                raise NotImplementedError("MultiscaleDiscriminator backward is not implemented yet: call under torch.no_grad()")
+        from . import autograd_g
+        with torch.set_grad_enabled(_records_grad(self, input)):
             return autograd_g.discriminator_forward_train(self, input)
-        with torch.no_grad():
-            a = ops.from_nchw(input.float())
-            result = []
-            ds = list(self.children())
-            for k, d in enumerate(ds):
-                outs = [o.to_nchw() for o in d.run(a)]
-                result.append(outs if not self.no_ganFeat_loss else [outs[-1]])
-                if k + 1 < len(ds):
-                    a = ops.avgpool3s2(a)
-            return result
 
 
 class GANLoss(nn.Module):

@@ -15,8 +15,8 @@ import torch.nn as nn
 from torch.nn.utils import spectral_norm
 
 from . import ops
-from .ops import ACT_LRELU, ACT_NONE, ACT_RELU, Act
-from .spade import _need_cuda, _param_key
+from .ops import ACT_RELU, Act
+from .spade import _need_cuda, _param_key, _records_grad
 
 
 def make_grid(N, iH, iW, opt=None):
@@ -297,59 +297,12 @@ class NLayerDiscriminator(nn.Module):
 
     def forward(self, input):
         _need_cuda(input, "NLayerDiscriminator")
-        with torch.no_grad():
-            seqs = ([getattr(self, "model" + str(i)) for i in range(self.n_layers + 2)] if self.getIntermFeat else [self.model])
-            outs = run_patch_sequences(seqs, ops.from_nchw(input.float()), self.training)
-            res = [o.to_nchw() for o in outs]
+        from . import autograd_g
+        seqs = [getattr(self, "model" + str(i)) for i in range(self.n_layers + 2)] if self.getIntermFeat else [self.model]
+        with torch.set_grad_enabled(_records_grad(self, input)):
+            outs = autograd_g.patchgan_forward(seqs, autograd_g.FromNCHW.apply(input.float(), None, None), self.training)
+            res = [autograd_g.nchw(o) for o in outs]
         return res if self.getIntermFeat else res[-1]
-
-
-def run_patch_sequences(seqs, a, training):
-    """Executes nn.Sequential containers made of {Conv2d 4x4 (s2|s1, pad 2), InstanceNorm2d, LeakyReLU, Dropout, Sigmoid}
-    with the kernels; returns one Act per container."""
-    from .spade import _conv_weight
-    outs = []
-    for seq in seqs:
-        mods = list(seq)
-        j = 0
-        while j < len(mods):
-            m = mods[j]
-            if isinstance(m, nn.Conv2d):
-                nxt = mods[j + 1:j + 3]
-                has_in = len(nxt) > 0 and isinstance(nxt[0], nn.InstanceNorm2d)
-                has_lr = any(isinstance(q, nn.LeakyReLU) for q in nxt[:2])
-                if len(nxt) > 0 and isinstance(nxt[0], nn.BatchNorm2d):
-                    raise NotImplementedError("BatchNorm discriminators have no kernel (reference uses norm='instance')")
-                w = _conv_weight(m, training)
-                bias = m.bias.detach().float().contiguous() if m.bias is not None else None
-                if m.stride[0] == 2:
-                    src = ops.space_to_depth(a)
-                    pw = ops.pack_s2d(w, 2)
-                    oh, ow = a.h // 2 + 1, a.w // 2 + 1
-                else:
-                    src, pw, oh, ow = a, ops.pack_weight(w, (2, 2)), a.h + 1, a.w + 1
-                cout = w.shape[0]
-                if cout == 1:
-                    o = Act.empty(a.n, oh, ow, 1, dtype=torch.float32, pitch=1)
-                    ops.conv2d(src, pw, o, shift=bias)
-                elif has_in:
-                    o = ops.conv2d(src, pw, Act.empty(a.n, oh, ow, cout), shift=bias)
-                    mean, rstd = ops.instnorm_stats(o, 0, None, oh, ow, None, None)
-                    ops.instnorm_apply(o, mean, rstd, ACT_LRELU if has_lr else ACT_NONE)
-                else:
-                    o = ops.conv2d(src, pw, Act.empty(a.n, oh, ow, cout), shift=bias, act=ACT_LRELU if has_lr else ACT_NONE)
-                a = o
-                j += 1 + int(has_in) + int(has_lr)
-            elif isinstance(m, nn.Dropout):
-                if training:
-                    raise NotImplementedError("Dropout in training mode is not implemented; call .eval()")
-                j += 1
-            elif isinstance(m, nn.Sigmoid):
-                raise NotImplementedError("use_sigmoid=True has no kernel (the reference uses LSGAN, use_sigmoid=False)")
-            else:
-                raise NotImplementedError("unexpected layer %s in a PatchGAN sequence" % type(m).__name__)
-        outs.append(a)
-    return outs
 
 
 class MultiscaleDiscriminator(nn.Module):
@@ -370,25 +323,10 @@ class MultiscaleDiscriminator(nn.Module):
 
     def forward(self, input):
         _need_cuda(input, "MultiscaleDiscriminator")
-        if torch.is_grad_enabled() and (input.requires_grad or any(p.requires_grad for p in self.parameters())) and not self.getIntermFeat:
-            # differentiable path (train_condition.py:208-232: D(fake) back-propagates into tocg, D(real/fake.detach()) into D)
-            from . import autograd_tocg
+        # train_condition.py:208-232: D(fake) back-propagates into tocg, D(real / fake.detach()) into D
+        from . import autograd_tocg
+        with torch.set_grad_enabled(_records_grad(self, input)):
             return autograd_tocg.tocg_discriminator_forward_train(self, input)
-        with torch.no_grad():
-            a = ops.from_nchw(input.float())
-            if self.Ddownx2:
-                a = ops.avgpool3s2(a)
-            result = []
-            for i in range(self.num_D):
-                k = self.num_D - 1 - i
-                if self.getIntermFeat:
-                    seqs = [getattr(self, "scale%d_layer%d" % (k, j)) for j in range(self.n_layers + 2)]
-                else:
-                    seqs = [getattr(self, "layer%d" % k)]
-                result.append([o.to_nchw() for o in run_patch_sequences(seqs, a, self.training)])
-                if i != self.num_D - 1:
-                    a = ops.avgpool3s2(a)
-            return result
 
 
 def weights_init(m):

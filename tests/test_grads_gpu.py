@@ -200,6 +200,40 @@ def test_tocg_discriminator_gradients():
     _check_d("tocg-D", res, res_ref, res_flo, grads, g_ref, g_flo)
 
 
+def test_tocg_discriminator_intermediate_features_are_differentiable():
+    """Stage-1 discriminator with getIntermFeat=True in train mode with grad enabled: every per-layer feature carries a gradient, and
+    the same layers, split into one sequence per layer group, compute what the flat getIntermFeat=False discriminator computes — the
+    logits and the weight gradients bit for bit."""
+    import contextlib
+    import io
+
+    import networks
+    seed = 37
+    with contextlib.redirect_stdout(io.StringIO()):
+        flat = networks.define_D(input_nc=33, Ddownx2=True, Ddropout=False, n_layers_D=3, spectral=False, num_D=2)
+        inter = networks.define_D(input_nc=33, Ddownx2=True, Ddropout=False, n_layers_D=3, spectral=False, num_D=2, getIntermFeat=True)
+    sd = {k: v.clone() for k, v in flat.state_dict().items()}
+    synth.fill_state_dict(sd, seed)
+    flat.load_state_dict(sd)
+    inter_keys = list(inter.state_dict())
+    assert len(inter_keys) == len(sd)
+    inter.load_state_dict(dict(zip(inter_keys, sd.values())))  # same layers in the same order: the keys map one to one
+    flat, inter = flat.cuda().train(), inter.cuda().train()
+    i1, i2 = synth.tocg_inputs(1, 256, 192, seed)
+    segs = synth.one_hot(synth.labels((1, 256, 192), 13, seed, "dseg"), 13)
+    inp = torch.cat([i1, i2, segs], 1).cuda()
+    res_flat, res_inter = flat(inp), inter(inp)
+    assert len(res_inter) == 2 and all(len(fs) == 5 for fs in res_inter)
+    assert all(f.requires_grad for fs in res_inter for f in fs)
+    for fs, (logits,) in zip(res_inter, res_flat):
+        assert torch.equal(fs[-1], logits)
+    for res in (res_flat, res_inter):
+        sum((fs[-1] * fs[-1]).mean() for fs in res).backward()
+    torch.cuda.synchronize()
+    for (name, p), (name_i, p_i) in zip(flat.named_parameters(), inter.named_parameters()):
+        assert p.grad is not None and torch.equal(p.grad, p_i.grad), (name, name_i)
+
+
 def test_stage2_train_step_runs():
     """One full stage-2 step (tocg -> warp -> G -> D -> hinge/feat/VGG -> Adam x2) at 512x384: finite losses, parameters move."""
     import types

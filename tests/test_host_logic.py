@@ -78,11 +78,12 @@ def test_tile_pickers():
 
 
 def test_s2d_weight_equivalence_on_cpu():
-    """The stride-2 -> space-to-depth rewrite is exact: conv(x, w, stride 2) == conv(s2d(x), s2d_weight(w), stride 1)."""
+    """The stride-2 -> space-to-depth rewrite is exact: conv(x, w, stride 2) == conv(s2d(x), s2d_weight(w), stride 1), and the
+    weight gradient of the rewritten convolution maps back onto the 4x4 / 3x3 parameter."""
     import torch.nn.functional as F
     for k, pad, h, w in [(4, 2, 11, 8), (3, 1, 10, 8), (3, 1, 9, 7), (4, 2, 12, 9)]:
         x = torch.randn(2, 5, h, w)
-        wt = torch.randn(6, 5, k, k)
+        wt = torch.randn(6, 5, k, k, requires_grad=True)
         ref = F.conv2d(x, wt, stride=2, padding=pad)
         c8 = 8
         xp = F.pad(x, (0, w % 2, 0, h % 2, 0, c8 - 5))
@@ -90,19 +91,23 @@ def test_s2d_weight_equivalence_on_cpu():
         s = xp.reshape(n, c, hh // 2, 2, ww // 2, 2).permute(0, 3, 5, 1, 2, 4).reshape(n, 4 * c, hh // 2, ww // 2)  # channel (py*2+px)*c8+ci
         got = F.conv2d(s, ops.s2d_weight(wt, pad), stride=1, padding=1)[:, :, :ref.shape[2], :ref.shape[3]]
         assert torch.allclose(got, ref, atol=1e-4), (k, pad, h, w)
+        got.square().sum().backward()
+        g1 = wt.grad.clone()
+        wt.grad = None
+        ref.square().sum().backward()
+        assert float((g1 - wt.grad).abs().max()) < 1e-3 * float(wt.grad.abs().max()), (k, pad, h, w)
 
 
 def test_im2col_weight_equivalence_on_cpu():
-    """autograd_g.im2col_weight: a 3x3 convolution over a few-channel map == a 1x1 convolution over the tap-major columns that
+    """ops.im2col_weight: a 3x3 convolution over a few-channel map == a 1x1 convolution over the tap-major columns that
     hrv_im2col produces (column j = tap*C + ci, zero padded to 64) — checked with F.unfold as the column builder."""
     import torch.nn.functional as F
-    from hrviton_b200 import autograd_g
     g = torch.Generator().manual_seed(0)
     x = torch.randn(2, 7, 9, 6, generator=g)
     w = torch.randn(12, 7, 3, 3, generator=g, requires_grad=True)
     cols = F.unfold(x, 3, padding=1).reshape(2, 7, 9, 9 * 6).permute(0, 2, 1, 3).reshape(2, 63, 9, 6)  # tap-major
     cols = F.pad(cols, (0, 0, 0, 0, 0, 1))
-    wc = autograd_g.im2col_weight(w, 64)
+    wc = ops.im2col_weight(w, 64)
     assert wc.shape == (12, 64, 1, 1)
     out = F.conv2d(cols, wc)
     ref = F.conv2d(x, w, padding=1)

@@ -352,7 +352,6 @@ def test_pack_conv_weight(dgrad, inter):
 @pytest.mark.parametrize("shape", [(2, 7, 12, 9), (1, 3, 8, 8)])
 def test_im2col_conv_equals_direct_conv(shape):
     """hrv_im2col + 1x1 GEMM == the 3x3 convolution it replaces (same products, fp32 accumulation)."""
-    from hrviton_b200 import autograd_g
     n, c, h, w = shape
     x = bf16r(synth.normalish(shape, 9, "x"))
     wt = bf16r(synth.normalish((24, c, 3, 3), 9, "w", 0.2))
@@ -361,7 +360,7 @@ def test_im2col_conv_equals_direct_conv(shape):
     unf = F.unfold(x, 3, padding=1).reshape(n, c, 9, h, w).permute(0, 3, 4, 2, 1).reshape(n, h, w, 9 * c)
     assert torch.equal(cols.buf[..., :9 * c].float().cpu(), unf)
     assert float(cols.buf[..., 9 * c:].float().abs().max()) == 0.0
-    wc = autograd_g.im2col_weight(wt.to(DEV), cols.c)
+    wc = ops.im2col_weight(wt.to(DEV), cols.c)
     out = Act.empty(n, h, w, 24)
     ops.conv2d(cols, ops.pack_weight(wc, (0, 0)), out)
     ref = F.conv2d(x, wt, padding=1)

@@ -43,7 +43,7 @@ for (h, w) in [(16, 12), (17, 13)]:
     y_ref = F.conv2d(x, wt, None, stride=2, padding=2); R = torch.randn_like(y_ref); (y_ref * R).sum().backward()
     x2 = x.detach().clone().requires_grad_(True); w2 = wt.detach().clone().requires_grad_(True)
     src = ag.space_to_depth_t(ag.FromNCHW.apply(x2, None, None))
-    y = ag.conv(src, ag._s2d_weight_t(w2), None, pad=1)
+    y = ag.conv(src, ops.s2d_weight(w2, 2), None, pad=1)
     y = y[:, :y_ref.shape[2], :y_ref.shape[3], :24].permute(0, 3, 1, 2).float()
     (y * R).sum().backward()
     print("s2d conv %dx%d: fwd %.2e dx %.2e dw %.2e" % (h, w, rel(y, y_ref), rel(x2.grad, x.grad), rel(w2.grad, wt.grad)))
@@ -74,11 +74,20 @@ for (h, w) in [(16, 12), (17, 13)]:
     y_ref = F.conv2d(x, wt, None, stride=2, padding=1); R = torch.randn_like(y_ref); (y_ref * R).sum().backward()
     x2 = x.detach().clone().requires_grad_(True); w2 = wt.detach().clone().requires_grad_(True)
     src = ag.space_to_depth_t(ag.FromNCHW.apply(x2, None, None))
-    y = ag.conv(src, ag._s2d_weight_t(w2), None, pad=1)
+    y = ag.conv(src, ops.s2d_weight(w2, 1), None, pad=1)
     y = y[:, :y_ref.shape[2], :y_ref.shape[3], :24].permute(0, 3, 1, 2).float()
     (y * R).sum().backward()
     print("s2d conv k3s2p1 %dx%d: fwd %.2e dx %.2e dw %.2e" % (h, w, rel(y, y_ref), rel(x2.grad, x.grad), rel(w2.grad, wt.grad)))
 # ---- bilinear x2 (+add) and the fused flow warp: kernel forward/backward vs torch autograd
+def warp_ref(src_nchw, flow_lo):
+    """networks.py:133-135 / 147-152 in torch: flow x2 (bilinear), normalise by ((W/2-1)/2,(H/2-1)/2), + base grid, grid_sample(border)."""
+    n, _, h, w = src_nchw.shape
+    fl = F.interpolate(flow_lo.permute(0, 3, 1, 2), scale_factor=2, mode="bilinear", align_corners=False).permute(0, 2, 3, 1)
+    fn = torch.cat([fl[..., 0:1] / ((w / 2 - 1.0) / 2.0), fl[..., 1:2] / ((h / 2 - 1.0) / 2.0)], 3)
+    gx = torch.linspace(-1.0, 1.0, w).view(1, 1, w, 1).expand(n, h, w, 1)
+    gy = torch.linspace(-1.0, 1.0, h).view(1, h, 1, 1).expand(n, h, w, 1)
+    grid = torch.cat([gx, gy], 3).to(src_nchw.device)
+    return F.grid_sample(src_nchw, fn + grid, mode="bilinear", padding_mode="border", align_corners=False), fl
 a = torch.randn(2, 24, 9, 7, device=dev).bfloat16().float().requires_grad_(True)
 b = torch.randn(2, 24, 18, 14, device=dev).bfloat16().float().requires_grad_(True)
 y_ref = F.interpolate(a, scale_factor=2, mode="bilinear", align_corners=False) + b; R = torch.randn_like(y_ref); (y_ref * R).sum().backward()
@@ -88,7 +97,7 @@ print("up2_add: fwd %.2e da %.2e db %.2e" % (rel(yn, y_ref), rel(a2.grad, a.grad
 for c in (48, 4):
     src = torch.randn(2, c, 32, 24, device=dev).bfloat16().float().requires_grad_(True)
     flow = (torch.randn(2, 16, 12, 2, device=dev) * 2.5).requires_grad_(True)
-    w_ref, fu_ref = at._warp(src, flow); R = torch.randn_like(w_ref); R2 = torch.randn_like(fu_ref)
+    w_ref, fu_ref = warp_ref(src, flow); R = torch.randn_like(w_ref); R2 = torch.randn_like(fu_ref)
     ((w_ref * R).sum() + (fu_ref * R2).sum()).backward()
     s2 = src.detach().clone().requires_grad_(True); f2 = flow.detach().clone().requires_grad_(True)
     wb, fu = at.FlowWarpFn.apply(ag.FromNCHW.apply(s2, None, None), f2)
